@@ -1,5 +1,5 @@
-"""Load the reference's OWN segmentor classes (staged byte-for-byte under ``baseline/_ref/py`` by
-``baseline/stage_ref.py``) on a chosen sparse backend.  Not product code: the product is the backend
+"""Load the reference's OWN segmentor classes (staged byte-for-byte under ``oracle/_ref/py`` by
+``oracle/stage_ref.py``) on a chosen sparse backend.  Not product code: the product is the backend
 under them; this is how tests and bench.py run the unmodified callers.
 
     ns = activate("b2s")        # torchsparse / range_utils / torch_scatter resolve to openpcseg_b200
@@ -24,7 +24,8 @@ import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-PY = os.path.join(HERE, "_ref", "py")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+PY = os.path.join(REF_DIR, "py")
 
 MODELS = {
     "minkunet34": ("voxel/semantic_kitti/minkunet_mk34_cr10.yaml",
@@ -60,8 +61,8 @@ def staged() -> bool:
 def _load_so(name: str, directory: str):
     hits = glob.glob(os.path.join(directory, name + ".*so"))
     if not hits:
-        raise FileNotFoundError(f"{name} is not built under {directory} (run baseline/stage_ref.py --cuda "
-                                f"or oracle/build_ref.py in the build container)")
+        raise FileNotFoundError(f"{name} is not built under {directory} (run oracle/stage_ref.py --cuda "
+                                f"or oracle/build_ref.py where the reference is available)")
     import torch  # noqa: F401  (libtorch first)
     spec = importlib.util.spec_from_file_location(name, hits[0])
     mod = importlib.util.module_from_spec(spec)
@@ -202,8 +203,8 @@ class Namespace:
 def activate(kind: str = "b2s") -> Namespace:
     assert kind in ("b2s", "ref_cuda", "ref_cpu"), kind
     if not staged():
-        raise FileNotFoundError("reference sources are not staged under baseline/_ref/py "
-                                "(python baseline/stage_ref.py in the build container)")
+        raise FileNotFoundError("reference sources are not staged under oracle/_ref/py "
+                                "(python oracle/stage_ref.py where the reference is available)")
     for name in [m for m in sys.modules if m.split(".")[0] in _PURGE]:
         del sys.modules[name]
     for p in (ROOT, PY):
@@ -219,10 +220,10 @@ def activate(kind: str = "b2s") -> Namespace:
         openpcseg_b200.install_as_torchsparse()
     else:
         if kind == "ref_cuda":
-            backend = _load_so("ts_ref_backend_cuda", os.path.join(HERE, "_ref"))
-            sys.modules["rangelib_cuda"] = _load_so("rangelib_cuda", os.path.join(HERE, "_ref"))
+            backend = _load_so("ts_ref_backend_cuda", REF_DIR)
+            sys.modules["rangelib_cuda"] = _load_so("rangelib_cuda", REF_DIR)
         else:
-            backend = _cpu_backend_proxy(_load_so("ts_ref_backend", os.path.join(ROOT, "oracle", "_ref")))
+            backend = _cpu_backend_proxy(_load_so("ts_ref_backend", REF_DIR))
             sys.modules["rangelib_cuda"] = _rangelib_cpu_standin()
         sys.modules["torchsparse.backend"] = backend
         sys.modules["torch_scatter"] = _torch_scatter_standin()

@@ -13,13 +13,13 @@ reference) over one batch of B synthetic SemanticKITTI-shaped scans (64 x 1875 r
                headline, as in round 1)
   --model-src  native     openpcseg_b200.segmentors.MinkUNet (same architecture / state_dict, BN+ReLU fused;
                           minkunet34 only, its default)
-               reference  the reference's OWN segmentor class, staged unmodified under baseline/_ref/py,
+               reference  the reference's OWN segmentor class, staged unmodified under oracle/_ref/py,
                           running on this backend through install_as_torchsparse() (default for the others)
   --impl       ours            this backend (libb2s) - the line the driver reads
                reference       the reference's own CPU implementation (its segmentor class on the CPU build of its
                                torchsparse, oracle/_ref) on host cores, bounded sub-scan per step, rank 0 only
                reference_cuda  the reference's own CUDA torchsparse recompiled for sm_100a
-                               (baseline/build_ref_cuda.py) under the same class, same GPU, same inputs
+                               (oracle/build_ref_cuda.py) under the same class, same GPU, same inputs
 
 Prints ONE JSON line:
   value         scans/s over all GPUs, inputs resident in HBM when the timed region starts
@@ -30,7 +30,7 @@ Prints ONE JSON line:
                 repeat of the same K steps after the `value` region
   cpu_baseline  the reference's CPU path on a bounded sub-scan (rank 0, N=1)
   ref_cuda      (N=1) the reference's CUDA build on the same workload, measured in the same run by a
-                child process of this script (--impl reference_cuda); None when baseline/_ref is absent
+                child process of this script (--impl reference_cuda); None when oracle/_ref has no CUDA build
   config1       (N=1) BASELINE configs[0]: one k3 submanifold conv on a 10 k-point cloud - naive PyTorch
                 gather-matmul-scatter on the host cores, the reference CPU backend, and this backend
 """
@@ -97,7 +97,13 @@ def parse():
     ap.add_argument("--cpu-budget-s", type=float, default=None,
                     help="CPU seconds for the reference arm (default 150 for --impl reference, 25 for the "
                          "cpu_baseline leg of the default run)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, take the timed step once more on the last timed step's batch from "
+                         "the run's starting state and write what it computed as DIR/<name>.npy (float32 / float64, "
+                         "fixed seeded samples of the large arrays; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.batch <= 0:
         args.batch = CONFIGS[args.config][1]
     if args.model_src is None:
@@ -325,10 +331,51 @@ def clocks_summary(proc):
             "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_LOGIT_ROWS = 1 << 18
+DUMP_PARAMS = 1 << 20
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, out: dict, model: torch.nn.Module) -> dict:
+    """Write the results of one training step as ``directory/<name>.npy`` so that two builds run with the same
+    arguments (hence the same inputs and initial weights) can be compared array by array:
+
+      loss    float64 [1]       the step's loss
+      logits  float32 [R, C]    the step's logits; R = all rows, or a fixed seeded sample of DUMP_LOGIT_ROWS rows
+                                (ascending row order) when there are more
+      params  float32 [P]       every parameter after the optimizer step, flattened and concatenated in
+                                ``model.parameters()`` order; a fixed seeded sample of DUMP_PARAMS elements
+                                (ascending index order) when there are more
+
+    The step dumped is the timed step function applied to the batch of the last timed step, starting from the
+    model, optimizer and loss-scaler state the run started from (seeded weights, no momentum): the kernels reduce
+    with float atomics, so the state reached after the warm-up and timed steps differs from run to run by more
+    than the rounding of one step.
+    """
+    g = torch.Generator().manual_seed(0)
+
+    def sample(n, k):
+        return torch.randperm(n, generator=g)[:k].sort().values if n > k else None
+
+    arrays = {"loss": out["loss"].detach().double().cpu().numpy().reshape(1)}
+    if "logits" in out:
+        y = out["logits"].detach().float()
+        rows = sample(y.shape[0], DUMP_LOGIT_ROWS)
+        arrays["logits"] = (y if rows is None else y[rows.to(y.device)]).cpu().numpy()
+    flat = torch.cat([p.detach().float().reshape(-1) for p in model.parameters()])
+    idx = sample(flat.numel(), DUMP_PARAMS)
+    arrays["params"] = (flat if idx is None else flat[idx.to(flat.device)]).cpu().numpy()
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    return {name: list(a.shape) for name, a in arrays.items()}
+
+
 def ref_cuda_child(args) -> dict | None:
     """Run ``--impl reference_cuda`` of the same config in a child process and return its JSON line."""
     import glob
-    if not glob.glob(os.path.join(ROOT, "baseline", "_ref", "ts_ref_backend_cuda.*so")):
+    if not glob.glob(os.path.join(ROOT, "oracle", "_ref", "ts_ref_backend_cuda.*so")):
         return None
     cmd = [sys.executable, os.path.abspath(__file__), "--impl", "reference_cuda", "--config", args.config,
            "--batch", str(args.batch), "--steps", str(min(args.steps, 6)), "--warmup", "3",
@@ -405,6 +452,9 @@ def main():
     # scaler.step() does not read it back (one host sync per step less; the same optimizer for both arms)
     opt = torch.optim.SGD(model.parameters(), lr=0.01, momentum=0.9, weight_decay=1e-4, fused=True)
     scaler = torch.amp.GradScaler("cuda", enabled=amp)
+    start_state = None
+    if args.dump_outputs:          # the state the dumped step starts from (see dump_outputs)
+        start_state = ({k: v.detach().clone() for k, v in model.state_dict().items()}, opt.state_dict())
 
     # ---- synthetic data: a pool of distinct batches per rank, in pinned host memory
     unit_key = "voxel_coord" if kind == "cylinder" else "coords"
@@ -418,14 +468,20 @@ def main():
     resident = [{k: v.to(dev) for k, v in p.items()} for p in pool]
     flush_buf = torch.empty(256 << 20, dtype=torch.uint8, device=dev)     # > 126 MB L2
 
+    last_out = {}                  # --dump-outputs: the results of the latest step
+
     def step(batch):
         opt.zero_grad(set_to_none=True)
         with torch.autocast("cuda", dtype=torch.float16, enabled=amp):
             if ns is None:
                 lidar = ts.SparseTensor(batch["feats"], batch["coords"], 1)
-                loss = net({"lidar": lidar, "targets": batch["labels"]})["loss"]
+                out = net({"lidar": lidar, "targets": batch["labels"]})
             else:
-                loss = net(ns.batch_dict(batch, dev))[0]["loss"]
+                out = net(ns.batch_dict(batch, dev))[0]
+        loss = out["loss"]
+        if args.dump_outputs:
+            last_out.clear()
+            last_out.update(out)
         scaler.scale(loss).backward()
         scaler.unscale_(opt)
         torch.nn.utils.clip_grad_norm_(model.parameters(), 10.0)
@@ -513,6 +569,18 @@ def main():
     # ---- timed region 2: end to end from pinned host buffers
     run(max(2, 2 * len(pool)), True)          # the copy stream has its own allocator pool: let it see every batch size
     ms_e2e, last_loss = run(args.steps, True)
+    dumped = None
+    if args.dump_outputs:          # every rank takes the step (DDP all-reduces its gradients), rank 0 writes it
+        model.load_state_dict(start_state[0])
+        opt.load_state_dict(start_state[1])
+        scaler = torch.amp.GradScaler("cuda", enabled=amp)
+        scale = scaler.get_scale()
+        torch.manual_seed(0)
+        step(resident[(args.steps - 1) % len(resident)])
+        torch.cuda.synchronize()
+        if rank == 0:
+            dumped = {"dir": args.dump_outputs, "shapes": dump_outputs(args.dump_outputs, last_out, model),
+                      "optimizer_step_applied": not amp or scaler.get_scale() >= scale}
 
     value = D.whole_job_rate(args.batch * args.steps, world, ms_dev)
     e2e = D.whole_job_rate(args.batch * args.steps, world, ms_e2e)
@@ -583,10 +651,12 @@ def main():
             "roofline": roof, "cpu_baseline": cpu_info}
     if not ours:
         line["impl"] = args.impl
-        line["config"]["backend"] = "reference torchsparse 1.4.0 CUDA backend recompiled for sm_100a (baseline/_ref)"
+        line["config"]["backend"] = "reference torchsparse 1.4.0 CUDA backend recompiled for sm_100a (oracle/_ref)"
     else:
         line["ref_cuda"] = ref_cuda
         line["config1"] = cfg1
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

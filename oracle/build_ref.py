@@ -55,7 +55,7 @@ _SPARSECONFIG = """\
 
 
 def module_path() -> str | None:
-    hits = glob.glob(os.path.join(OUT_DIR, MOD_NAME + "*.so"))
+    hits = glob.glob(os.path.join(OUT_DIR, MOD_NAME + ".*so"))     # not ts_ref_backend_cuda
     return hits[0] if hits else None
 
 

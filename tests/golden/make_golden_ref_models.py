@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Run the reference's OWN four sparse segmentors (staged unmodified by baseline/stage_ref.py) on the CPU
+"""Run the reference's OWN four sparse segmentors (staged unmodified by oracle/stage_ref.py) on the CPU
 build of its bundled torchsparse (oracle/_ref) and freeze their outputs (build container only).
 
     python tests/golden/make_golden_ref_models.py  ->  tests/golden/ref_models.npz

@@ -46,7 +46,7 @@ def test_model_batches_have_the_reference_collate_layout():
     assert c["offset"][-1] == len(c["voxel_coord"]) == len(c["voxel_label"])
 
 
-@pytest.mark.skipif(not loader.staged(), reason="baseline/_ref/py not staged (build container step)")
+@pytest.mark.skipif(not loader.staged(), reason="oracle/_ref/py not staged (the reference is not available)")
 @pytest.mark.parametrize("name,kind,n_params,n_conv", CASES)
 def test_reference_segmentors_construct_unmodified_on_the_shim(name, kind, n_params, n_conv):
     ns = loader.activate("b2s")
